@@ -249,6 +249,17 @@ def cpu_reference_rate(pairs, budget_s, max_regs, all_cores=False):
     return done / dt, (min(cores, workers * per_reg) if all_cores else min(cores, workers * 3)), done, dt
 
 
+def dump_outputs(out_dir, results, prefix):
+    """Writes the per-pair results of one batch call as out_dir/<prefix><field>.npy, one row per pair: what a caller
+    of the call receives, in float64 (float32 where the ABI's field is a float), so that two builds can be compared
+    output for output on the benchmark's seeded inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    fields = {"T": np.float64, "info": np.float64, "sigma": np.float32, "confidence": np.float32, "code": np.float64,
+              "iters": np.float64, "n_corr": np.float64, "n_src": np.float64}
+    for name, dtype in fields.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), np.array([r[name] for r in results], dtype=dtype))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -269,7 +280,13 @@ def main():
     ap.add_argument("--clock-sampler", default="smi", choices=["nvml", "smi", "off"],
                     help="how SM clocks / throttle reasons are sampled during the timed regions: NVML in-process, "
                          "the profiling recipe's nvidia-smi -lms 200 process (default), or not at all (A/B of the sampler's own cost: none measured)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's results of the last timed step (T, info, sigma, confidence, "
+                         "code, iters, n_corr, n_src per pair; about 0.5 KB per pair) as DIR/<field>.npy for the "
+                         "device-resident value leg and DIR/e2e_<field>.npy for the end-to-end leg")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of the GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -424,7 +441,7 @@ def main():
         best_pipe.run_resident()
         barrier()
         f0, f1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        k20 = max(2, min(args.steps, 5))
+        k20 = args.steps
         f0.record()
         r20, _ = best_pipe.run_resident_steps(k20)
         f1.record()
@@ -538,6 +555,9 @@ def main():
     errs = [synth.pose_error(r["T"], p["T_gt"]) for r, p in zip(res, pairs)]
     ok = all(r["code"] == 1 for r in res) and max(e[0] for e in errs) < 0.05
     assert ok, ("registration failed inside the benchmark", [r["code"] for r in res], errs)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res_p, "")
+        dump_outputs(args.dump_outputs, res_e2e, "e2e_")
 
     # ---- reduce over ranks -------------------------------------------------------------------
     dev_s = dev_ms / 1e3

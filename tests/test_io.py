@@ -1,10 +1,14 @@
 """On-disk formats (SURVEY 8f rank 3): PCD / KITTI .bin readers into the ABI's AoS48 layout, pose writer."""
+import hashlib
 import os
 
 import numpy as np
 import pytest
 
 from mulls_b200 import io as mio
+
+DEMO_PCD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "demo_000000_head.pcd")
+DEMO_PCD_ROWS_SHA256 = "a86107f2ea8e9b8885df7e1df072a91d6061519b70d139259ef3c772691af73b"
 
 
 def _write_pcd(path, arr, fields, binary=True):
@@ -69,11 +73,13 @@ def test_pose_writer(tmp_path):
     assert len(vals) == 12 and vals[3] == 1.2345679 and vals[7] == -2.5 and vals[11] == 1e-9
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/demo_data/pcd/000000.pcd"), reason="reference demo data not present")
 def test_reads_reference_demo_scan():
-    c = mio.read_pcd("/root/reference/demo_data/pcd/000000.pcd")
-    assert c.shape == (124668, 12)
+    """The first 4096 points of MULLS's demo scan 000000 (tests/golden/make_golden_pcd.py): the rows must be what the
+    reader made of the original 124 668-point file."""
+    c = mio.read_pcd(DEMO_PCD)
+    assert c.shape == (4096, 12)
     assert abs(np.linalg.norm(c[:1000, 4:7], axis=1) - 1.0).max() < 1e-3
+    assert hashlib.sha256(c.tobytes()).hexdigest() == DEMO_PCD_ROWS_SHA256
 
 
 # ---- the native readers of the C-ABI (csrc/scan_io.h) against the numpy ones above: bit for bit -------------------
@@ -133,8 +139,7 @@ def test_native_reader_errors_and_pose_writer(tmp_path):
     assert open(a).read() == open(b).read()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/demo_data/pcd/000000.pcd"), reason="reference demo data not present")
 def test_native_reader_on_the_reference_demo_scan():
-    a = mio.read_pcd("/root/reference/demo_data/pcd/000000.pcd")
-    b = mio.read_cloud_block_native("/root/reference/demo_data/pcd/000000.pcd")
+    a = mio.read_pcd(DEMO_PCD)
+    b = mio.read_cloud_block_native(DEMO_PCD)
     np.testing.assert_array_equal(b["pc_raw"].view(np.uint32), a.view(np.uint32))
