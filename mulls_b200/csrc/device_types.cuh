@@ -13,8 +13,6 @@ constexpr int kNumSegs = 2 * kNumClasses; // seg = side*6 + class; side 0 = targ
 constexpr int kIterBlock = 128;           // threads (= source points) per iteration-kernel block
 constexpr int kIngestBlock = 256;         // input points per ingest block
 constexpr int kTerms = 28;                // 21 lower-tri ATPA + 6 ATPb (+1 pad) per class partial
-constexpr int kMaxLevels = 12;
-constexpr int kCoordBits = 12;            // Morton bits per axis
 constexpr int kDedupMinSrc = 500;         // K_filter_distant_point (cregistration.hpp:1704)
 constexpr unsigned kClaimFree = 0x7f7f7f7fu;
 constexpr int kIterFlags = 256;           // per-iteration stop flags kept for the launch loop of sharded runs

@@ -16,6 +16,8 @@
 namespace mulls {
 
 constexpr uint32_t kKeyHiMask = 0xffffu;
+constexpr int kMaxLevels = 12; // levels 0 .. 11: the top level has 2 x 2 x 2 cells, the whole grid
+constexpr int kCoordBits = 12; // Morton bits per axis: 4096 level-0 cells
 
 // FLANN L2_Simple<float> accumulation (result += diff*diff per axis, float) — the distance the reference's
 // kd-tree returns to CorrespondenceEstimation (cregistration.hpp:1745). Non-fused: the library is built with

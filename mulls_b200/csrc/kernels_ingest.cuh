@@ -165,17 +165,13 @@ __global__ void k_pair_setup(DeviceArrays A, int n_pairs, float h0_min) {
         }
         ext = fmax(ext, gmax[d] - gmin[d]);
     }
-    const int ncell = 1 << kCoordBits;
-    float h0 = h0_min;
-    while ((ext + 8.0 * h0) * 1.001 > (double)h0 * (ncell - 4)) h0 *= 2.0f;
+    const float h0 = grid_h0(ext, h0_min); // (search_core.cuh)
     ps.h0 = h0;
     ps.inv_h0 = 1.0f / h0; // power of two times h0_min: exact when h0_min is a power of two
     for (int d = 0; d < 3; ++d) ps.origin[d] = (float)gmin[d] - 2.0f * h0;
-    // number of levels: the top level's guaranteed coverage 0.999*h must reach the largest search
-    // radius 2.5*dis_thre_unit (filter_dis_times, cregistration.hpp:1707)
-    const float rmax = 2.5f * pc.thre_unit * 1.0001f;
-    int L = 2; // level l's 2x2x2 block covers 0.999 * h0 * 2^(l-1) (see nn_search)
-    while (L < kMaxLevels && 0.999f * 0.5f * h0 * (float)(1 << (L - 1)) < rmax) ++L;
+    // number of levels: the top level's guaranteed coverage 0.999 * h_top / 2 must reach the largest search radius
+    // 2.5 * thre that the threshold schedule reaches in max_iter iterations (grid_levels, search_core.cuh)
+    int L = grid_levels(h0, pc.thre_unit, pc.thre_min, pc.thre_rate, pc.max_iter);
     // normal shooting needs the exact 10 nearest targets with no distance bound: full pyramid, whose top 2x2x2
     // block (2 x 2048 level-0 cells per axis) spans the whole grid
     if (pc.normal_shooting) L = kMaxLevels;

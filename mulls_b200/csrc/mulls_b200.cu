@@ -479,7 +479,10 @@ int mulls_set_tunable(mulls_ctx *ctx, const char *name, int value) {
         ctx->stage_wc = value;
     }
     else if (n == "pack_threads") PackPool::get().ensure_workers(value);
-    else if (n == "h0_min_mm") ctx->h0_min = (float)value / 1000.0f;
+    else if (n == "h0_min_mm") {
+        if (value <= 0) return MULLS_E_ARG; // (grid_h0 doubles it until the cloud fits)
+        ctx->h0_min = (float)value / 1000.0f;
+    }
     else return MULLS_E_ARG;
     return MULLS_OK;
 }
@@ -587,6 +590,13 @@ static void setup_undistortion(const double *m, PairConst &pc) {
 static int build_pair_const(mulls_ctx *ctx, const mulls_icp_params &P, const double *init, PairConst &pc) {
     if (P.max_iter_num > MULLS_MAX_TRACE_ITERS) {
         ctx->err = "max_iter_num > 64";
+        return MULLS_E_ARG;
+    }
+    // the threshold schedule sizes the search grid (grid_levels) and bounds every search radius
+    if (!(std::isfinite(P.dis_thre_unit) && P.dis_thre_unit > 0.0f) ||
+        !(std::isfinite(P.dis_thre_update_rate) && P.dis_thre_update_rate > 0.0f) ||
+        !(std::isfinite(P.dis_thre_min) && P.dis_thre_min >= 0.0f)) {
+        ctx->err = "dis_thre_unit and dis_thre_update_rate must be finite and > 0, dis_thre_min finite and >= 0";
         return MULLS_E_ARG;
     }
     std::memset(&pc, 0, sizeof(pc));

@@ -20,6 +20,7 @@
 //            carries the mask of existing children, the children that can still beat the bound are pushed with their
 //            box distance — and a small cell is examined where it is met (or, once the seeds are good, queued and
 //            examined together with the block's other small cells in one go)
+//            The top level of the full pyramid (2x2x2 cells) takes all 8 cells: the block is the whole grid
 //   stop     best <= cover_l^2 (the best found is the global nearest) or cover_l^2 >= r2_prune; else next level
 //   scan     a small cell's points four at a time: fused estimates of the squared distances, their minimum against the
 //            best so far, and only then the exact FLANN distances with the tie rule (walk_scan_leaf)
@@ -56,6 +57,34 @@ struct GridView {
     int leaf_count; // cells with at most this many points are scanned, larger ones are split
     float level_slack2; // >= 1.002001: the start level's coverage must reach sqrt(level_slack2) x the seed distance
 };
+
+// ---- grid geometry of one pair (k_pair_setup; tests/harness/search_host.cu exports both rules to the CPU suite) ----
+// level-0 cell size: h0_min, doubled until the extent plus two cells of margin on each side fits in 4096 - 4 cells
+MULLS_HD float grid_h0(double ext, float h0_min) {
+    float h0 = h0_min;
+    while ((ext + 8.0 * h0) * 1.001 > (double)h0 * ((1 << kCoordBits) - 4)) h0 *= 2.0f;
+    return h0;
+}
+
+// number of levels: the top level's guaranteed coverage 0.999 * h_top / 2 (nn_search_walk) must reach the largest search
+// radius 2.5 * thre (filter_dis_times, cregistration.hpp:1707) of any iteration. solve_and_advance updates the threshold
+// as thre <- max(thre / rate, thre_min) from thre_unit, so it grows when rate < 1 or thre_min > thre_unit; the largest
+// value of iterations 0 .. max_iter - 1 is followed here in double (the float updates round by at most 64 half ulps,
+// far inside the 1.0001 of rmax). A shrinking schedule gives thre_unit itself, bit for bit. Beyond the coverage of the
+// full pyramid there is nothing left to add: its top level is the whole grid (nn_search_walk examines all 8 cells).
+MULLS_HD int grid_levels(float h0, float thre_unit, float thre_min, float thre_rate, int max_iter) {
+    float thre_max = thre_unit;
+    double t = (double)thre_unit;
+    for (int k = 1; k < max_iter; ++k) {
+        t = t / (double)thre_rate;
+        if (!(t > (double)thre_min)) t = (double)thre_min;
+        if (t > (double)thre_max) thre_max = (float)t;
+    }
+    const float rmax = 2.5f * thre_max * 1.0001f;
+    int L = 2; // level l's 2x2x2 block covers 0.999 * h0 * 2^(l-1)
+    while (L < kMaxLevels && 0.999f * 0.5f * h0 * (float)(1 << (L - 1)) < rmax) ++L;
+    return L;
+}
 
 struct NoStats {
     MULLS_HD void probe() {}
@@ -330,10 +359,14 @@ MULLS_HD float nn_search_walk_b(const GridView &g, float px, float py, float pz,
     for (;; ++l) {
         st.level();
         const float H = g.h0 * (float)(1 << l);
-        const int ncell = 4096 >> l;
+        const int ncell = (1 << kCoordBits) >> l;
+        const bool whole = ncell == 2; // top of the full pyramid: its 8 cells ARE the grid, all of them are walked
         int xs[2], ys[2], zs[2];
         xs[0] = c0x >> l, ys[0] = c0y >> l, zs[0] = c0z >> l;
-        if (l == 0) { // side of the half-cell p lies in: by the fractional position inside the level-0 cell
+        if (whole) { // p's own cell first where p is inside the grid
+            xs[0] = (xs[0] > 0) ? 1 : 0, ys[0] = (ys[0] > 0) ? 1 : 0, zs[0] = (zs[0] > 0) ? 1 : 0;
+            xs[1] = xs[0] ^ 1, ys[1] = ys[0] ^ 1, zs[1] = zs[0] ^ 1;
+        } else if (l == 0) { // side of the half-cell p lies in: by the fractional position inside the level-0 cell
             xs[1] = xs[0] + (((fx - flx) >= 0.5f) ? 1 : -1);
             ys[1] = ys[0] + (((fy - fly) >= 0.5f) ? 1 : -1);
             zs[1] = zs[0] + (((fz - flz) >= 0.5f) ? 1 : -1);
@@ -351,8 +384,14 @@ MULLS_HD float nn_search_walk_b(const GridView &g, float px, float py, float pz,
             vz[i] = zs[i] >= 0 && zs[i] < ncell;
         }
         // p lies inside its own cell (the margin covers the rounding of the cell assignment): only the three
-        // neighbour slabs are at a distance
+        // neighbour slabs are at a distance — except on the whole grid, whose first cells are only the nearest ones
         ex[0] = ey[0] = ez[0] = 0.0f;
+        if (whole) {
+            ex[0] = walk_axis_dist(g.ox, H, xs[0], px, margin);
+            ey[0] = walk_axis_dist(g.oy, H, ys[0], py, margin);
+            ez[0] = walk_axis_dist(g.oz, H, zs[0], pz, margin);
+            ex[0] *= ex[0], ey[0] *= ey[0], ez[0] *= ez[0];
+        }
         ex[1] = walk_axis_dist(g.ox, H, xs[1], px, margin);
         ey[1] = walk_axis_dist(g.oy, H, ys[1], py, margin);
         ez[1] = walk_axis_dist(g.oz, H, zs[1], pz, margin);
@@ -450,9 +489,12 @@ MULLS_HD float nn_search_walk_b(const GridView &g, float px, float py, float pz,
             walk_scan_leaf(g, px, py, pz, q_start[qi], q_count[qi], best_d2, best_j, wb);
         }
         nq = 0;
-        const float cover = (l == 0) ? 0.998f * 0.5f * g.h0 : 0.999f * 0.5f * H; // every closer target has been examined
+        // every closer target has been examined (the whole grid: every target has been examined or pruned)
+        const float cover = whole ? INFINITY : (l == 0) ? 0.998f * 0.5f * g.h0 : 0.999f * 0.5f * H;
         const float cover2 = cover * cover;
-        // every target outside the block is farther than `cover`; inside it, what was not examined is behind `pruned`
+        // every target outside the block is farther than `cover`; inside it, what was not examined is behind `pruned`.
+        // Stopping at a top level below the full pyramid relies on grid_levels: its coverage reaches every radius the
+        // pair searches with
         if (best_d2 <= cover2 || cover2 >= r2_prune || l == L - 1) // (global nearest found / whole radius examined / top)
             return wb.radius2(cover2);
     }

@@ -48,7 +48,8 @@ void insert(HostGrid &G, uint32_t x, uint32_t y, uint32_t z, int level, uint32_t
 
 extern "C" {
 
-// pts: n x 4 floats (x y z _). Grid geometry as k_pair_setup would choose it is supplied by the caller.
+// pts: n x 4 floats (x y z _). Grid geometry as k_pair_setup would choose it (sh_h0_for, sh_levels_for) is supplied by
+// the caller.
 void *sh_build(const float *pts, uint32_t n, float ox, float oy, float oz, float h0, int n_levels, int leaf_count) {
     HostGrid *G = new HostGrid();
     std::vector<uint64_t> key(n);
@@ -167,6 +168,12 @@ int sh_search(void *h, const float *q, const int *seed, uint32_t m, float r2_pru
               int *out_idx, float *out_d2, uint64_t *stats /*[12]*/, uint32_t *evals_per_query /*[m] or null*/) {
     return sh_search_cert(h, q, seed, m, r2_prune, start_level, reseed_d2, out_idx, out_d2, stats, evals_per_query, nullptr);
 }
+
+// the grid geometry rules of k_pair_setup (search_core.cuh)
+int sh_levels_for(float h0, float thre_unit, float thre_min, float thre_rate, int max_iter) {
+    return grid_levels(h0, thre_unit, thre_min, thre_rate, max_iter);
+}
+float sh_h0_for(double ext, float h0_min) { return grid_h0(ext, h0_min); }
 
 uint32_t sh_morton_roundtrip(uint32_t v) { return compact12(spread12(v)) == (v & 0xfffu) && compact12(spread12(v) << 1 >> 1) == (v & 0xfffu); }
 

@@ -32,25 +32,24 @@ def lib():
     lb.sh_search.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_float, C.c_int, C.c_float, C.c_void_p,
                              C.c_void_p, C.c_void_p, C.c_void_p]
     lb.sh_search_cert.argtypes = lb.sh_search.argtypes + [C.c_void_p]
+    lb.sh_levels_for.restype = C.c_int
+    lb.sh_levels_for.argtypes = [C.c_float, C.c_float, C.c_float, C.c_float, C.c_int]
+    lb.sh_h0_for.restype = C.c_float
+    lb.sh_h0_for.argtypes = [C.c_double, C.c_float]
     lb.sh_morton_roundtrip.restype = C.c_uint32
     lb.sh_morton_roundtrip.argtypes = [C.c_uint32]
     return lb
 
 
-def n_levels(h0, radius):
-    L = 2
-    while L < 12 and 0.999 * 0.5 * h0 * (1 << (L - 1)) < radius * 1.0001:
-        L += 1
-    return L
-
-
-def run(lib, tgt_xyz, q_xyz, radius, seeds=None, leaf=32, h0=0.125, reseed=-1.0, mode=0, want_cert=False):
+def run(lib, tgt_xyz, q_xyz, radius, seeds=None, leaf=32, h0=0.125, reseed=-1.0, mode=0, want_cert=False, levels=None):
+    """search every query within `radius` on a grid of level-0 cell size h0; `levels` defaults to what k_pair_setup
+    chooses when `radius` is the largest radius of the pair (2.5 x dis_thre_unit, a shrinking schedule)"""
     tgt_xyz = np.ascontiguousarray(tgt_xyz, np.float32)
     q_xyz = np.ascontiguousarray(q_xyz, np.float32)
     origin = (tgt_xyz.min(0) - 2 * h0).astype(np.float32)
     pts4 = np.ascontiguousarray(np.concatenate([tgt_xyz, np.zeros((len(tgt_xyz), 1), np.float32)], axis=1))
     G = lib.sh_build(pts4.ctypes.data, len(tgt_xyz), float(origin[0]), float(origin[1]), float(origin[2]), h0,
-                     n_levels(h0, radius), leaf)
+                     levels if levels is not None else lib.sh_levels_for(h0, radius / 2.5, 0.0, 2.0, 1), leaf)
     m = len(q_xyz)
     idx = np.empty(m, np.int32)
     d2 = np.empty(m, np.float32)
