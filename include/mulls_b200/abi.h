@@ -470,7 +470,18 @@ int mulls_pose_write(const char *path, const double pose[16], int overwrite);
 void *mulls_host_alloc(size_t bytes);
 void mulls_host_free(void *p);
 
-/* Runtime tunables (integers), e.g. "start_level", "pairs_in_flight". Returns MULLS_E_ARG if unknown. */
+/* Runtime tunables (integers). A pipelined context passes them to its lanes, a context to the twin it double-buffers
+ * one-shot batches with.
+ *   "leaf_count"    search-grid cells with at most this many points are scanned, larger ones are split (default 32)
+ *   "hash_slack"    grid hash tables hold at least hash_slack x cells entries; values below 2 count as 2 (default 4)
+ *   "h0_min_mm"     smallest level-0 grid cell edge in mm, > 0 (default 125)
+ *   "use_graph"     1: the iteration loop runs as one CUDA graph or, for small batches, as k_icp_loop; 0: the host
+ *                   launch loop, one launch per kernel (default 1)
+ *   "loop_kernel"   1: small batches run the whole loop as one cooperative kernel (k_icp_loop); 0: never (default 1)
+ *   "host_pack"     host clouds cross PCIe packed to 28 B/point: 0 never, 1 always, 2 when a call ships at least 2^18
+ *                   points (default 2)
+ *   "pack_threads"  grow the process-wide packing pool to this many workers
+ * Returns MULLS_E_ARG for an unknown name or a value outside the ranges above. */
 int mulls_set_tunable(mulls_ctx *ctx, const char *name, int value);
 
 #ifdef __cplusplus

@@ -53,8 +53,8 @@ struct PairConst {
     double tbound[6];           // block1->local_bound
     // layout
     uint32_t in_off[kNumSegs];  // offset (points) of each input cloud in the AoS48 staging array
-    const float4 *in_ptr[kNumSegs]; // where the ingest kernel reads the cloud: the HBM copy, or (one-shot calls with
-                                    // pinned host buffers) the caller's buffer itself, streamed over PCIe (zero-copy)
+    const float4 *in_ptr[kNumSegs]; // where the ingest kernel reads the cloud: the HBM copy, or (targets from a
+                                    // device-resident local map) the map's own buffer
     uint32_t in_n[kNumSegs];
     uint32_t in_fmt[kNumSegs];  // layout behind in_ptr: 0 = 48-byte rows, 1 = packed 16+12 B, 2 = packed 16+16 B (host_pack.h)
     uint32_t tgt_base[kNumClasses]; // base of each class in the target SoA arrays (capacity = in_n)

@@ -202,7 +202,7 @@ __global__ void k_pair_setup(DeviceArrays A, int n_pairs, float h0_min) {
 
 // ---- k_make_keys: intersection filter (cfilter.hpp:950-981: strictly inside) + 64-bit sort key
 //      [pair*12+seg | morton36(cell)]; filtered-out points sort to the very end.
-__global__ void __launch_bounds__(kIngestBlock) k_make_keys(DeviceArrays A, int sort_sources) {
+__global__ void __launch_bounds__(kIngestBlock) k_make_keys(DeviceArrays A) {
     const ChunkDesc cd = A.in_chunks[blockIdx.x];
     const PairConst &pc = A.pc[cd.pair];
     PairState &ps = A.ps[cd.pair];
@@ -228,8 +228,6 @@ __global__ void __launch_bounds__(kIngestBlock) k_make_keys(DeviceArrays A, int 
             cy = min(max(cy, 0), hi);
             cz = min(max(cz, 0), hi);
             key = ((uint64_t)(cd.pair * kNumSegs + seg) << 36) | morton36((uint32_t)cx, (uint32_t)cy, (uint32_t)cz);
-            // (study switch: sources left in the caller's order — nothing but the search's locality depends on it)
-            if (!sort_sources && seg >= kNumClasses) key = ((uint64_t)(cd.pair * kNumSegs + seg) << 36) | (uint64_t)local;
         }
         A.keys_a[gi] = key;
         A.vals_a[gi] = (uint32_t)gi;

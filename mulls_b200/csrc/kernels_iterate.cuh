@@ -236,10 +236,14 @@ __device__ __forceinline__ bool shoots(const PairConst &pc, int c) {
 //   0.37 / 0.28 / 0.16 for iterations 3 / 4 / 5; the queue interleaves chunks, and the locality of a warp's 32 queries
 //   is worth more than its density.)
 constexpr int kKeepFromIter = 3;
+// search parameters (profiles/r2_search_ab_scan4_occupancy.txt: other deferral iterations and reseed distances are
+// no faster)
+constexpr int kStartLevel = 5;       // grid level at which a walk starts
+constexpr int kDeferFromIter = 3;    // from this iteration on a block queues its small cells (one scan loop per block)
+constexpr float kReseedCells = 4.0f; // a previous match farther than this many level-0 cells is challenged by a greedy descent
 
 struct SearchArgs {
-    int start_level0, leaf_count, defer_from_iter;
-    float reseed_cells;
+    int leaf_count;
 };
 
 // what is fixed for all queries of one (pair, class): grid, radius
@@ -255,7 +259,7 @@ __device__ __forceinline__ SearchFrame search_frame(const DeviceArrays &A, const
     const float max_distance_f = 2.5f * ps.thre;
     f.max_dist_sqr = (double)max_distance_f * (double)max_distance_f;
     f.r2_prune = (float)f.max_dist_sqr * 1.0001f;
-    f.defer = ps.iter >= sa.defer_from_iter; // queueing a block's small cells pays once the seeds are good
+    f.defer = ps.iter >= kDeferFromIter; // queueing a block's small cells pays once the seeds are good
     return f;
 }
 
@@ -276,7 +280,7 @@ __device__ __forceinline__ void search_finish(DeviceArrays &A, const PairConst &
 // match that the last increment left far away (the big first corrections) is challenged by a fresh greedy descent.
 template <class Bounds>
 __device__ __forceinline__ void search_one(DeviceArrays &A, const PairConst &pc, int c, int buf, uint32_t gi, const float4 p,
-                                           float orig_bits, const SearchFrame &f, const SearchArgs &sa, bool write_cert) {
+                                           float orig_bits, const SearchFrame &f, bool write_cert) {
     NoStats st;
     int best_j = -1;
     float best_d2 = INFINITY;
@@ -287,15 +291,15 @@ __device__ __forceinline__ void search_one(DeviceArrays &A, const PairConst &pc,
         best_j = pj;
     }
     {
-        const float rs = sa.reseed_cells * f.g.h0;
+        const float rs = kReseedCells * f.g.h0;
         if (best_j < 0 || best_d2 > rs * rs) {
             float d2 = INFINITY;
             int j = -1;
-            walk_greedy_seed(f.g, p.x, p.y, p.z, sa.start_level0, d2, j, st);
+            walk_greedy_seed(f.g, p.x, p.y, p.z, kStartLevel, d2, j, st);
             if (j >= 0 && d2 < best_d2) best_d2 = d2, best_j = j;
         }
     }
-    const float cert2 = nn_search_walk_b<Bounds>(f.g, p.x, p.y, p.z, f.r2_prune, sa.start_level0, f.defer, best_d2, best_j, st);
+    const float cert2 = nn_search_walk_b<Bounds>(f.g, p.x, p.y, p.z, f.r2_prune, kStartLevel, f.defer, best_d2, best_j, st);
     if (write_cert) A.src_cert[buf][gi] = make_float4(p.x, p.y, p.z, sqrtf(cert2));
     search_finish(A, pc, c, gi, best_j, best_d2, f.max_dist_sqr, orig_bits);
 }
@@ -324,7 +328,7 @@ __device__ __forceinline__ void search_quarter(DeviceArrays &A, int buf, uint32_
         return;
     }
     const SearchFrame f = search_frame(A, pc, ps, c, sa);
-    search_one<Bounds>(A, pc, c, buf, gi, p, n.w, f, sa, write_cert);
+    search_one<Bounds>(A, pc, c, buf, gi, p, n.w, f, write_cert);
 }
 
 // keep mode: one block, one chunk. need_list / n_need live in shared memory.
@@ -383,7 +387,7 @@ __device__ __forceinline__ void search_keep_chunk(DeviceArrays &A, int buf, uint
     if (threadIdx.x < *n_need) {
         const uint32_t gi = pc.src_base[c] + cd.first + need_list[threadIdx.x];
         const float4 p = A.src_pos[buf][gi]; // (advanced by pass A)
-        search_one<WalkBounds>(A, pc, c, buf, gi, p, A.src_nrm[buf][gi].w, f, sa, true);
+        search_one<WalkBounds>(A, pc, c, buf, gi, p, A.src_nrm[buf][gi].w, f, true);
     }
 }
 
@@ -393,8 +397,7 @@ constexpr int kSearchBlocksPerSm = 12; // 40 registers (measured against 10 / 16
 __device__ __forceinline__ int search_mode_of(int it) { return it >= kKeepFromIter ? 2 : (it == kKeepFromIter - 1 ? 1 : 0); }
 
 template <int kMode>
-__global__ void __launch_bounds__(kIterBlock, kSearchBlocksPerSm) k_search(DeviceArrays A, int buf, int it, int start_level0, int leaf_count,
-                                                                          int defer_from_iter, float reseed_cells) {
+__global__ void __launch_bounds__(kIterBlock, kSearchBlocksPerSm) k_search(DeviceArrays A, int buf, int it, int leaf_count) {
     buf = loop_buf(A, buf);
     if (it < 0) it = A.ctl->it; // (graph: the device-side loop counter; every running pair is in this iteration)
     if (blockIdx.x == 0 && threadIdx.x == 0) { // first kernel(s) of the iteration: counters and list the later ones use
@@ -403,7 +406,7 @@ __global__ void __launch_bounds__(kIterBlock, kSearchBlocksPerSm) k_search(Devic
         ctl.n_live[buf ^ 1] = 0u;
     }
     if (search_mode_of(it) != kMode) return;
-    const SearchArgs sa = {start_level0, leaf_count, defer_from_iter, reseed_cells};
+    const SearchArgs sa = {leaf_count};
     if (kMode == 2) {
         __shared__ uint8_t s_need[kIterBlock];
         __shared__ uint32_t s_n_need;
@@ -427,7 +430,7 @@ __global__ void __launch_bounds__(kIterBlock, kSearchBlocksPerSm) k_search(Devic
 // the one with the smallest squared distance to the line through the source point along its normal; dropped
 // if that value exceeds max_distance (NOT squared); correspondence distance = its squared NN distance.
 // Launched only when a pair of the batch asked for normal shooting.
-__device__ __forceinline__ void search_shoot_chunk(DeviceArrays &A, int buf, uint32_t chunk, int start_level0, int leaf_count) {
+__device__ __forceinline__ void search_shoot_chunk(DeviceArrays &A, int buf, uint32_t chunk, int leaf_count) {
     const ChunkDesc cd = A.it_chunks[chunk];
     const PairConst &pc = A.pc[cd.pair];
     const PairState &ps = A.ps[cd.pair];
@@ -451,7 +454,7 @@ __device__ __forceinline__ void search_shoot_chunk(DeviceArrays &A, int buf, uin
     int sj = -1;
     float sd2 = INFINITY;
     KnnList kl;
-    knn_search(g, p.x, p.y, p.z, start_level0, kl);
+    knn_search(g, p.x, p.y, p.z, kStartLevel, kl);
     double min_dist = 1.7976931348623157e308;
     for (int t = 0; t < kl.n; ++t) {
         const float4 q = __ldg(&g.pos[kl.j[t]]);
@@ -470,9 +473,9 @@ __device__ __forceinline__ void search_shoot_chunk(DeviceArrays &A, int buf, uin
     A.nn_idx[gi] = sj;
     A.nn_d2[gi] = sd2;
 }
-__global__ void __launch_bounds__(kIterBlock) k_search_shoot(DeviceArrays A, int buf, int start_level0, int leaf_count) {
+__global__ void __launch_bounds__(kIterBlock) k_search_shoot(DeviceArrays A, int buf, int leaf_count) {
     buf = loop_buf(A, buf);
-    for_each_live_chunk(A, buf, 3, [&](uint32_t chunk) { search_shoot_chunk(A, buf, chunk, start_level0, leaf_count); });
+    for_each_live_chunk(A, buf, 3, [&](uint32_t chunk) { search_shoot_chunk(A, buf, chunk, leaf_count); });
 }
 
 // ---- k_resolve ---------------------------------------------------------------------------------
@@ -1087,12 +1090,11 @@ __global__ void __launch_bounds__(kSolveThreads) k_solve(DeviceArrays A, int buf
 //      phases are the same device functions over the same work lists, separated by grid-wide barriers instead of kernel
 //      boundaries. Every block executes the same number of barriers: the loop bounds (LoopCtl::max_iter, the running
 //      counter read after a barrier) are grid-uniform.
-__global__ void __launch_bounds__(kIterBlock, 4) k_icp_loop(DeviceArrays A, int start_level0, int leaf_count, int defer_from_iter,
-                                                           float reseed_cells) {
+__global__ void __launch_bounds__(kIterBlock, 4) k_icp_loop(DeviceArrays A, int leaf_count) {
     namespace cg = cooperative_groups;
     cg::grid_group grid = cg::this_grid();
     LoopCtl &ctl = *A.ctl;
-    const SearchArgs sa = {start_level0, leaf_count, defer_from_iter, reseed_cells};
+    const SearchArgs sa = {leaf_count};
     __shared__ uint8_t s_need[kIterBlock];
     __shared__ uint32_t s_n_need;
     const int n_pairs = ctl.n_pairs, max_iter = ctl.max_iter;
@@ -1374,8 +1376,8 @@ __global__ void k_finalize(DeviceArrays A, int n_pairs) {
 
 // ---- k_nn_query: mulls_nn_query — exact 1-NN of arbitrary query points in one target class of pair 0, on the grid
 //      the last registration built (what block1->tree_*->nearestKSearch(p, 1) answers in the reference)
-__global__ void __launch_bounds__(kIterBlock) k_nn_query(DeviceArrays A, int cls, const float *xyz, uint32_t n, int start_level0,
-                                                        int leaf_count, int *out_idx, float *out_d2) {
+__global__ void __launch_bounds__(kIterBlock) k_nn_query(DeviceArrays A, int cls, const float *xyz, uint32_t n, int leaf_count,
+                                                        int *out_idx, float *out_d2) {
     const uint32_t i = blockIdx.x * kIterBlock + threadIdx.x;
     if (i >= n) return;
     const PairConst &pc = A.pc[0];
@@ -1388,8 +1390,8 @@ __global__ void __launch_bounds__(kIterBlock) k_nn_query(DeviceArrays A, int cls
         const float rmax = 2.5f * pc.thre_unit;
         const float r2 = rmax * rmax * 1.0001f;
         NoStats st;
-        walk_greedy_seed(g, px, py, pz, start_level0, best_d2, best_j, st);
-        nn_search_walk(g, px, py, pz, r2, start_level0, false, best_d2, best_j, st);
+        walk_greedy_seed(g, px, py, pz, kStartLevel, best_d2, best_j, st);
+        nn_search_walk(g, px, py, pz, r2, kStartLevel, false, best_d2, best_j, st);
         if (best_j >= 0 && !((double)best_d2 <= (double)rmax * (double)rmax)) best_j = -1;
         if (best_j >= 0) best_j = __float_as_int(__ldg(&g.nrm[best_j]).w);
     }

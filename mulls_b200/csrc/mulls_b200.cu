@@ -99,34 +99,29 @@ struct mulls_ctx {
     void *nccl_comm = nullptr; // ncclComm_t created by mulls_nccl_init (destroyed with the context)
     bool any_keep_less = false;
     bool grid_valid = false; // pair 0's sorted target slices and grid are those of the last registration (mulls_nn_query)
-    // tunables
-    int start_level0 = 5;
-    int leaf_count = 32;
+    // tunables (mulls_set_tunable)
+    struct Tunables {
+        int leaf_count = 32;    // grid cells with at most this many points are scanned, larger ones are split
+        int hash_slack = 4;     // table capacity >= hash_slack x cells (power of two): load factor <= 1/hash_slack
+        float h0_min = 0.125f;  // smallest level-0 cell edge (m); grid_h0 doubles it until the cloud fits
+        int use_graph = 1;      // 1: the iteration graph (or k_icp_loop); 0: the host launch loop (per-kernel events)
+        int loop_kernel = 1;    // small batches: the whole iteration loop as one cooperative kernel (k_icp_loop)
+        // repack host clouds to the 28 B/point wire format on the host cores before the DMA (host_pack.h):
+        // 0 never, 1 always, 2 when a call ships at least kPackMinPoints points (small calls are latency-bound: raw rows)
+        int host_pack = 2;
+    } tun;
     // iteration loop as a CUDA graph: WHILE(pairs running) { search, resolve, accumulate, solve } + posterior, finalize,
-    // collect — one launch, the loop condition is set on the device (no host polling). Built on first use, rebuilt when a
-    // tunable baked into its kernel nodes changes. 0: the host launch loop (per-kernel events for the bench's roofline).
-    int use_graph = 1;
+    // collect — one launch, the loop condition is set on the device (no host polling). Built on first use, rebuilt when
+    // what is baked into its kernel nodes changes.
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t graph_exec = nullptr;
-    int graph_key[6] = {-1, -1, -1, -1, -1, -1}; // the tunables baked into the kernel nodes
+    int graph_key[3] = {-1, -1, -1}; // what is baked into the kernel nodes (build_iteration_graph)
     LoopCtl *h_ctl = nullptr;            // pinned staging of the control block
     int num_sms = 148;
-    int sort_sources = 1;    // 0: sources stay in the caller's order (study switch)
-    int search_blocks = 12;  // resident k_search blocks per SM (10 / 12 / 16: register budget 48 / 40 / 32; measured 4.36 / 4.31 / 4.61 ms of search per 64-pair step)
-    int defer_from_iter = 3; // k_search queues the small cells of a block (one scan loop per block) from this iteration on
-    int hash_slack = 4;      // table capacity >= hash_slack x cells (power of two): load factor <= 1/hash_slack
-    int reseed_cells_x4 = 16; // a previous match farther than this many quarter level-0 cells is challenged by a greedy descent
     bool any_normal_shooting = false;
     bool any_undistort = false;
-    int zero_copy = 0;     // opt-in: one-shot calls read pinned host clouds in place (measured slower than DMA: 20 vs 32 GB/s)
-    // repack host clouds to the 28 B/point wire format on the host cores before the DMA (host_pack.h):
-    // 0 never, 1 always, 2 when a call ships at least kPackMinPoints points (small calls are latency-bound: raw rows)
-    int host_pack = 2;
-    int poll_pause = 64;   // _mm_pause() count between two cudaEventQuery calls of the launch loop's flow control
-    int stage_wc = 0;      // allocate the pinned staging write-combined (the host only streams into it)
     float4 *h_stage = nullptr; // pinned staging of the packed clouds (allocated on first use)
     size_t h_stage_slots = 0;
-    float h0_min = 0.125f;
     // timing
     cudaEvent_t ev_begin = nullptr, ev_ingest = nullptr, ev_iter = nullptr, ev_end = nullptr, ev_h2d0 = nullptr;
     bool h2d_timed = false;                 // ev_h2d0 was recorded by the upload of the current one-shot call
@@ -141,8 +136,6 @@ struct mulls_ctx {
     // one-shot batch calls with host buffers (mulls_icp_run_batch) are double-buffered: the second half of the batch is
     // packed and copied on the twin's stream while the first half is being registered on this one
     mulls_ctx *twin = nullptr;
-    int double_buffer = 1;
-    int loop_kernel = 1;       // small batches: the whole iteration loop as one cooperative kernel (k_icp_loop)
     int loop_kernel_blocks = 0; // co-resident blocks of k_icp_loop on this device (0: not yet queried, -1: unavailable)
     struct Pending {                 // a run that has been enqueued and not yet finished (run_finish)
         uint64_t launches = 0;
@@ -456,33 +449,15 @@ int mulls_set_tunable(mulls_ctx *ctx, const char *name, int value) {
         const int rc = mulls_set_tunable(ctx->twin, name, value);
         if (rc != MULLS_OK) return rc;
     }
-    std::string n(name);
-    if (n == "start_level") ctx->start_level0 = value;
-    else if (n == "leaf_count") ctx->leaf_count = value;
-    else if (n == "reseed_cells_x4") ctx->reseed_cells_x4 = value;
-    else if (n == "defer_from_iter") ctx->defer_from_iter = value;
-    else if (n == "search_blocks") ctx->search_blocks = value; // (kept for old scripts: the instantiations are fixed now)
-    else if (n == "sort_sources") ctx->sort_sources = value;
-    else if (n == "double_buffer") ctx->double_buffer = value;
-    else if (n == "loop_kernel") ctx->loop_kernel = value;
-    else if (n == "hash_slack") ctx->hash_slack = std::max(2, value);
-    else if (n == "use_graph") ctx->use_graph = value;
-    else if (n == "zero_copy") ctx->zero_copy = value;
-    else if (n == "host_pack") ctx->host_pack = value;
-    else if (n == "poll_pause") ctx->poll_pause = value;
-    else if (n == "stage_wc") {
-        if (ctx->stage_wc != value && ctx->h_stage) { // re-allocated with the new flag on the next packed upload
-            cudaFreeHost(ctx->h_stage);
-            ctx->h_stage = nullptr;
-            ctx->h_stage_slots = 0;
-        }
-        ctx->stage_wc = value;
-    }
-    else if (n == "pack_threads") PackPool::get().ensure_workers(value);
-    else if (n == "h0_min_mm") {
-        if (value <= 0) return MULLS_E_ARG; // (grid_h0 doubles it until the cloud fits)
-        ctx->h0_min = (float)value / 1000.0f;
-    }
+    mulls_ctx::Tunables &t = ctx->tun;
+    const std::string n(name);
+    if (n == "leaf_count") t.leaf_count = value;
+    else if (n == "hash_slack") t.hash_slack = std::max(2, value);
+    else if (n == "h0_min_mm" && value > 0) t.h0_min = (float)value / 1000.0f;
+    else if (n == "use_graph" && (value == 0 || value == 1)) t.use_graph = value;
+    else if (n == "loop_kernel" && (value == 0 || value == 1)) t.loop_kernel = value;
+    else if (n == "host_pack" && value >= 0 && value <= 2) t.host_pack = value;
+    else if (n == "pack_threads") PackPool::get().ensure_workers(value); // (process-wide)
     else return MULLS_E_ARG;
     return MULLS_OK;
 }
@@ -635,9 +610,9 @@ static int build_pair_const(mulls_ctx *ctx, const mulls_icp_params &P, const dou
     return MULLS_OK;
 }
 
-// resident = true: the clouds are copied into HBM (mulls_batch_upload: they must survive the caller's buffers).
-// resident = false (one-shot calls): clouds in PINNED host memory are not copied at all — the ingest kernel
-// streams them over PCIe itself (zero-copy through the UVA alias), pageable ones are staged with cudaMemcpy.
+// The clouds are copied into HBM (a device-resident local map as target is read in place). resident = true
+// (mulls_batch_upload): the call returns once the copies are done. resident = false (one-shot calls): it returns with
+// the copies in flight, and run_impl, which follows at once, synchronises before it returns.
 static int upload_impl(mulls_ctx *ctx, size_t n_pairs, const mulls_cloud_view *tgt, const mulls_cloud_view *src,
                        const mulls_icp_params *params, const double *init_guess, const uint32_t *src_index_base,
                        const uint32_t *src_global_n, bool resident = true, bool tgt_on_device = false) {
@@ -708,20 +683,18 @@ static int upload_impl(mulls_ctx *ctx, size_t n_pairs, const mulls_cloud_view *t
         ctx->err = "internal: chunk table capacity";
         return MULLS_E_CAPACITY;
     }
-    // the clouds: repacked on the host cores and copied pair by pair (host_pack), or copied as they are, or read in
-    // place (zero-copy, pinned host buffers of one-shot calls)
+    // the clouds: repacked on the host cores and copied pair by pair (host_pack), or copied as they are
     size_t host_points = 0;
     for (size_t p = 0; p < n_pairs; ++p)
         for (int s = 0; s < kNumSegs; ++s)
             if (!(tgt_on_device && s < kNumClasses)) host_points += ctx->h_pc[p].in_n[s];
     const size_t kPackMinPoints = 1u << 18;
     bool tables_sent = false;
-    const bool pack = ctx->host_pack == 1 || (ctx->host_pack == 2 && host_points >= kPackMinPoints);
+    const bool pack = ctx->tun.host_pack == 1 || (ctx->tun.host_pack == 2 && host_points >= kPackMinPoints);
     if (pack) {
         if (!ctx->h_stage) {
             const size_t slots = 2 * ctx->cap_in + 4 * kNumSegs * ctx->max_pairs;
-            CK(cudaHostAlloc((void **)&ctx->h_stage, slots * sizeof(float4),
-                             ctx->stage_wc ? cudaHostAllocWriteCombined : cudaHostAllocDefault));
+            CK(cudaHostAlloc((void **)&ctx->h_stage, slots * sizeof(float4), cudaHostAllocDefault));
             ctx->h_stage_slots = slots;
         }
         CK(cudaStreamSynchronize(ctx->stream)); // the staging may still be read by a copy of a call that failed half-way
@@ -796,15 +769,6 @@ static int upload_impl(mulls_ctx *ctx, size_t n_pairs, const mulls_cloud_view *t
                 pc.in_ptr[s] = (const float4 *)v.aos48;
                 continue;
             }
-            if (!resident && ctx->zero_copy) {
-                cudaPointerAttributes attr;
-                if (cudaPointerGetAttributes(&attr, v.aos48) == cudaSuccess && attr.type == cudaMemoryTypeHost &&
-                    attr.devicePointer != nullptr && ((uintptr_t)attr.devicePointer % 16) == 0) {
-                    pc.in_ptr[s] = (const float4 *)attr.devicePointer;
-                    continue;
-                }
-                cudaGetLastError(); // pageable memory: not an error, fall through to the copy
-            }
             CK(cudaMemcpyAsync((void *)(ctx->A.in_aos + 3 * (size_t)pc.in_off[s]), v.aos48, v.n * 48, cudaMemcpyHostToDevice,
                                ctx->stream));
         }
@@ -863,10 +827,10 @@ static int launch_ingest(mulls_ctx *ctx, DeviceArrays &A, bool trace, uint64_t &
         k_shard_pack_setup<<<1, 1, 0, st>>>(A, 1);
         launches += 2;
     }
-    k_pair_setup<<<(unsigned)ceil_div(np, 128), 128, 0, st>>>(A, np, ctx->h0_min);
+    k_pair_setup<<<(unsigned)ceil_div(np, 128), 128, 0, st>>>(A, np, ctx->tun.h0_min);
     ++launches;
     if (n_inc) {
-        k_make_keys<<<n_inc, kIngestBlock, 0, st>>>(A, ctx->sort_sources);
+        k_make_keys<<<n_inc, kIngestBlock, 0, st>>>(A);
         ++launches;
         if (ctx->any_keep_less) { // random down-sampling of :2866-2892: radix select of the k-th sampling key
             const unsigned pb = (unsigned)ceil_div(np, 64);
@@ -900,13 +864,13 @@ static int launch_ingest(mulls_ctx *ctx, DeviceArrays &A, bool trace, uint64_t &
         k_gather<<<(unsigned)ceil_div(n_in, 256), 256, 0, st>>>(A, A.keys_b, A.vals_b, n_in);
         const unsigned hb = (unsigned)ceil_div((size_t)n_in + 1, 256);
         k_hash_build<<<hb, 256, 0, st>>>(A, A.keys_b, n_in, 0);
-        k_hash_layout<<<1, 32, 0, st>>>(A, np, ctx->hash_slack);
+        k_hash_layout<<<1, 32, 0, st>>>(A, np, ctx->tun.hash_slack);
         k_hash_clear<<<1184, 256, 0, st>>>(A);
         k_hash_build<<<hb, 256, 0, st>>>(A, A.keys_b, n_in, 1);
         k_hash_build<<<hb, 256, 0, st>>>(A, A.keys_b, n_in, 2);
         launches += 6;
     } else {
-        k_hash_layout<<<1, 32, 0, st>>>(A, np, ctx->hash_slack);
+        k_hash_layout<<<1, 32, 0, st>>>(A, np, ctx->tun.hash_slack);
         ++launches;
     }
     return MULLS_OK;
@@ -926,12 +890,12 @@ static unsigned resident_grid(const mulls_ctx *ctx, int blocks_per_sm) {
 // it < 0 (recording the iteration graph): all three modes, each checks the device-side iteration counter; the host
 // launch loop knows the iteration and launches the one that runs
 static void launch_search(mulls_ctx *ctx, cudaStream_t st, const DeviceArrays &A, int buf, int it) {
-    const float reseed = 0.25f * (float)ctx->reseed_cells_x4;
+    const int leaf = ctx->tun.leaf_count;
     const unsigned grid = resident_grid(ctx, kSearchBlocksPerSm);
     const int mode = it < 0 ? -1 : (it >= kKeepFromIter ? 2 : (it == kKeepFromIter - 1 ? 1 : 0));
-    if (mode < 0 || mode == 0) k_search<0><<<grid, kIterBlock, 0, st>>>(A, buf, it, ctx->start_level0, ctx->leaf_count, ctx->defer_from_iter, reseed);
-    if (mode < 0 || mode == 1) k_search<1><<<grid, kIterBlock, 0, st>>>(A, buf, it, ctx->start_level0, ctx->leaf_count, ctx->defer_from_iter, reseed);
-    if (mode < 0 || mode == 2) k_search<2><<<grid, kIterBlock, 0, st>>>(A, buf, it, ctx->start_level0, ctx->leaf_count, ctx->defer_from_iter, reseed);
+    if (mode < 0 || mode == 0) k_search<0><<<grid, kIterBlock, 0, st>>>(A, buf, it, leaf);
+    if (mode < 0 || mode == 1) k_search<1><<<grid, kIterBlock, 0, st>>>(A, buf, it, leaf);
+    if (mode < 0 || mode == 2) k_search<2><<<grid, kIterBlock, 0, st>>>(A, buf, it, leaf);
 }
 constexpr int kShootBlocksPerSm = 8, kResolveBlocksPerSm = 16, kAccumulateBlocksPerSm = 8;
 
@@ -940,8 +904,7 @@ constexpr int kShootBlocksPerSm = 8, kResolveBlocksPerSm = 16, kAccumulateBlocks
 // context with grids sized for its capacity; what a run needs to know (chunk / pair counts, trace switch, loop counter)
 // is read from LoopCtl in device memory. k_solve's last block sets the loop condition: no host polling, one launch.
 static int build_iteration_graph(mulls_ctx *ctx) {
-    const int key[6] = {ctx->start_level0, ctx->leaf_count + (ctx->reseed_cells_x4 << 12), (int)chunk_bucket(ctx),
-                        ctx->any_normal_shooting ? 1 : 0, ctx->defer_from_iter, ctx->search_blocks};
+    const int key[3] = {ctx->tun.leaf_count, (int)chunk_bucket(ctx), ctx->any_normal_shooting ? 1 : 0};
     if (ctx->graph_exec && std::memcmp(key, ctx->graph_key, sizeof(key)) == 0) return MULLS_OK;
     if (ctx->graph_exec) cudaGraphExecDestroy(ctx->graph_exec), ctx->graph_exec = nullptr;
     if (ctx->graph) cudaGraphDestroy(ctx->graph), ctx->graph = nullptr;
@@ -961,7 +924,7 @@ static int build_iteration_graph(mulls_ctx *ctx) {
     CK(cudaStreamBeginCaptureToGraph(st, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
     launch_search(ctx, st, A, -1, -1);
     if (ctx->any_normal_shooting)
-        k_search_shoot<<<resident_grid(ctx, kShootBlocksPerSm), kIterBlock, 0, st>>>(A, -1, ctx->start_level0, ctx->leaf_count);
+        k_search_shoot<<<resident_grid(ctx, kShootBlocksPerSm), kIterBlock, 0, st>>>(A, -1, ctx->tun.leaf_count);
     k_resolve<<<resident_grid(ctx, kResolveBlocksPerSm), kIterBlock, 0, st>>>(A, -1);
     k_accumulate<<<resident_grid(ctx, kAccumulateBlocksPerSm), kIterBlock, 0, st>>>(A, -1);
     k_solve<<<cap_pairs, kSolveThreads, 0, st>>>(A, -1, (unsigned long long)handle);
@@ -1022,7 +985,7 @@ static int run_impl_inner(mulls_ctx *ctx, mulls_icp_result *out, mulls_icp_trace
     }
     // small batches: one cooperative kernel runs the whole loop (every chunk and every pair must find a co-resident block)
     bool looped = false;
-    if (!hook && ctx->use_graph && ctx->loop_kernel && !ctx->any_normal_shooting && n_itc > 0) {
+    if (!hook && ctx->tun.use_graph && ctx->tun.loop_kernel && !ctx->any_normal_shooting && n_itc > 0) {
         if (ctx->loop_kernel_blocks == 0) {
             int per_sm = 0, coop = 0;
             cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, ctx->device);
@@ -1031,11 +994,9 @@ static int run_impl_inner(mulls_ctx *ctx, mulls_icp_result *out, mulls_icp_trace
             else
                 ctx->loop_kernel_blocks = -1, cudaGetLastError();
         }
-        // `loop_kernel` = how many chunks a co-resident block may have to walk per phase (1: every chunk has its block)
-        looped = ctx->loop_kernel_blocks > 0 && n_itc <= (unsigned)(ctx->loop_kernel * ctx->loop_kernel_blocks) &&
-                 np <= ctx->loop_kernel * ctx->loop_kernel_blocks;
+        looped = ctx->loop_kernel_blocks > 0 && n_itc <= (unsigned)ctx->loop_kernel_blocks && np <= ctx->loop_kernel_blocks;
     }
-    const bool graphed = !hook && ctx->use_graph && !looped;
+    const bool graphed = !hook && ctx->tun.use_graph && !looped;
     if (graphed) {
         const int rc = build_iteration_graph(ctx);
         if (rc != MULLS_OK) return rc;
@@ -1044,9 +1005,8 @@ static int run_impl_inner(mulls_ctx *ctx, mulls_icp_result *out, mulls_icp_trace
     int n_search_ev = 0;
     if (looped) {
         DeviceArrays Aarg = A;
-        int a1 = ctx->start_level0, a2 = ctx->leaf_count, a3 = ctx->defer_from_iter;
-        float a4 = 0.25f * (float)ctx->reseed_cells_x4;
-        void *args[] = {&Aarg, &a1, &a2, &a3, &a4};
+        int leaf = ctx->tun.leaf_count;
+        void *args[] = {&Aarg, &leaf};
         const unsigned grid = std::max(1u, std::min((unsigned)ctx->loop_kernel_blocks, std::max(n_itc, (unsigned)np)));
         CK(cudaLaunchCooperativeKernel((const void *)k_icp_loop, dim3(grid), dim3(kIterBlock), args, 0, st));
         k_posterior<<<n_itc, kIterBlock, 0, st>>>(A);
@@ -1061,8 +1021,9 @@ static int run_impl_inner(mulls_ctx *ctx, mulls_icp_result *out, mulls_icp_trace
             // as every pair has converged or failed (the device mirrors its counter into mapped memory)
             if (it >= 2) {
                 // (poll with pauses: several lanes spinning inside the driver slow each other's launches down)
+                constexpr int kPollPause = 64;
                 while (cudaEventQuery(ctx->ev_done[it - 2]) == cudaErrorNotReady)
-                    for (int k = 0; k < ctx->poll_pause; ++k) _mm_pause();
+                    for (int k = 0; k < kPollPause; ++k) _mm_pause();
                 // Sharded runs must take this decision identically on every rank (the ranks issue matching collectives):
                 // they read the count the device recorded at the END of iteration it-2 — written once, before
                 // ev_done[it-2] — never the live flag, whose value at this instant depends on each rank's timing.
@@ -1076,7 +1037,7 @@ static int run_impl_inner(mulls_ctx *ctx, mulls_icp_result *out, mulls_icp_trace
             CK(cudaEventRecord(ctx->ev_search[2 * it], st));
             launch_search(ctx, st, A, buf, it);
             if (ctx->any_normal_shooting) {
-                k_search_shoot<<<resident_grid(ctx, kShootBlocksPerSm), kIterBlock, 0, st>>>(A, buf, ctx->start_level0, ctx->leaf_count);
+                k_search_shoot<<<resident_grid(ctx, kShootBlocksPerSm), kIterBlock, 0, st>>>(A, buf, ctx->tun.leaf_count);
                 ++launches;
             }
             CK(cudaEventRecord(ctx->ev_search[2 * it + 1], st));
@@ -1222,14 +1183,11 @@ int mulls_batch_run_resident(mulls_ctx *ctx, mulls_icp_result *out, mulls_icp_tr
 static int one_shot_batch(mulls_ctx *ctx, size_t n_pairs, const mulls_cloud_view *tgt, const mulls_cloud_view *src,
                           const mulls_icp_params *params, const double *init_guess, mulls_icp_result *out, mulls_icp_trace *trace) {
     const double t0 = wall_ms();
-    const bool split = ctx->double_buffer && ctx->use_graph && n_pairs >= 2 && n_pairs <= ctx->max_pairs;
+    const bool split = ctx->tun.use_graph && n_pairs >= 2 && n_pairs <= ctx->max_pairs;
     if (split && !ctx->twin) {
         mulls_ctx *t = mulls_create(ctx->device, (ctx->max_pairs + 1) / 2, ctx->max_src, ctx->max_tgt);
         if (t) { // (no memory for it: the call simply runs on one context)
-            t->start_level0 = ctx->start_level0, t->leaf_count = ctx->leaf_count, t->reseed_cells_x4 = ctx->reseed_cells_x4;
-            t->defer_from_iter = ctx->defer_from_iter, t->sort_sources = ctx->sort_sources, t->hash_slack = ctx->hash_slack;
-            t->use_graph = ctx->use_graph, t->zero_copy = ctx->zero_copy, t->host_pack = ctx->host_pack, t->poll_pause = ctx->poll_pause;
-            t->stage_wc = ctx->stage_wc, t->h0_min = ctx->h0_min, t->double_buffer = 0;
+            t->tun = ctx->tun;
             ctx->twin = t;
         }
     }
@@ -1370,8 +1328,7 @@ int mulls_nn_query(mulls_ctx *ctx, int cls, const float *xyz, size_t n, int32_t 
     CK(cudaMallocAsync((void **)&d_i, n * sizeof(int), st));
     CK(cudaMallocAsync((void **)&d_d, n * sizeof(float), st));
     CK(cudaMemcpyAsync(d_q, xyz, 3 * n * sizeof(float), cudaMemcpyHostToDevice, st));
-    k_nn_query<<<(unsigned)ceil_div(n, kIterBlock), kIterBlock, 0, st>>>(ctx->A, cls, d_q, (uint32_t)n, ctx->start_level0,
-                                                                           ctx->leaf_count, d_i, d_d);
+    k_nn_query<<<(unsigned)ceil_div(n, kIterBlock), kIterBlock, 0, st>>>(ctx->A, cls, d_q, (uint32_t)n, ctx->tun.leaf_count, d_i, d_d);
     CK(cudaMemcpyAsync(idx, d_i, n * sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(d2, d_d, n * sizeof(float), cudaMemcpyDeviceToHost, st));
     cudaFreeAsync(d_q, st);

@@ -24,9 +24,9 @@ small["tgt"] = downsample(full["tgt"], (9000, 2000, 7000, 2000, 0, 0), 2)    # <
 p = abi.IcpParams.from_buffer_copy(full["params"]); p.used_feature_type = b"111100"; p.target_bound[:] = synth.cloud_bound(small["tgt"])
 small["params"] = p
 cases["slam operating point 2.6k/20k"] = small
-for name, pair in [(n + m, p) for n, p in cases.items() for m in ("", " [host launch loop]", " [iteration graph]", " [loop kernel x2]", " [loop kernel x4]")]:
+for name, pair in [(n + m, p) for n, p in cases.items() for m in ("", " [host launch loop]", " [iteration graph]")]:
     ctx.set_tunable("use_graph", 0 if "host launch loop" in name else 1)
-    ctx.set_tunable("loop_kernel", 0 if "iteration graph" in name else (2 if "x2" in name else (4 if "x4" in name else 1)))
+    ctx.set_tunable("loop_kernel", 0 if "iteration graph" in name else 1)
     for _ in range(3): res, _ = ctx.run_batch([pair])
     t0 = time.perf_counter(); n = 20
     for _ in range(n): res, _ = ctx.run_batch([pair])

@@ -1,6 +1,6 @@
 """A/B of search tunables in ONE process on ONE box: the same resident batch, per-iteration device time of the
 search launch (host launch loop, CUDA events), for a list of tunable settings.
-    python scripts/gpu_search_ab.py <pairs> <config> "dfs_until=0" "dfs_until=20" "dfs_until=2" ..."""
+    python scripts/gpu_search_ab.py <pairs> <config> "leaf_count=32" "leaf_count=24" "leaf_count=48" ..."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from concurrent.futures import ProcessPoolExecutor
